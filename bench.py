@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - participant-steps/s of the batched env.step() hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the fused tick (physics -> pose -> collisions -> out-of-bound -> status) over one
@@ -107,6 +107,25 @@ def make_scene_name(config: str) -> str:
     return {"c2": f"C2 {N_SCN}x{M_PART} kinematics + OBB collision, synthetic grid map",
             "c3": "C3 4096x64 dynamics + map polylines", "c4": "C4 16384x32 mixed vehicle/cyclist/pedestrian",
             "c5": "C5 65536x128 kinematics + broadphase stress"}[config]
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """Write `arrays` (each with the scenario axis first) to `path`/<name>.npy as float32, the integer outputs converted
+    exactly, plus scenario_index.npy (float64): the scenario rows written.  When the whole batch would exceed DUMP_BYTES,
+    a fixed seeded sample of scenario rows is written, the same rows for every array, so that two builds run with the
+    same arguments can be compared array by array."""
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(a[0].size for a in arrays.values()) * 4 + 8
+    keep = min(n, (DUMP_BYTES - (64 << 10)) // row_bytes)          # 64 KiB left for the .npy headers
+    rows = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, f"{k}.npy"), a[rows].astype(np.float32))
+    np.save(os.path.join(path, "scenario_index.npy"), rows.astype(np.float64))
+    print(f"[bench] wrote {len(arrays) + 1} arrays ({keep} of {n} scenarios) to {path}", file=sys.stderr)
 
 
 class ClockSampler:
@@ -471,6 +490,12 @@ def run_ours(args):
             break
     t_wall1 = time.time()
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    if args.dump_outputs and rank == 0:
+        # every repetition restores the worlds first, so the last timed step's results do not depend on how many ran
+        last = worlds[(K - 1) % R]
+        outs = {k: getattr(last, k) for k in ("x", "y", "heading", "speed", "vx", "vy")}
+        outs.update({k: getattr(last.result, k) for k in ("flags", "hit_index", "hit_segment", "status", "done")})
+        dump_outputs(args.dump_outputs, {k: v.cpu().numpy() for k, v in outs.items()})
     ms_total = float(np.median(reps_ms))
     ms_per_step = ms_total / K
     value = world_size * n * m * K / (ms_total * 1e-3)
@@ -652,7 +677,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned (rank 0's "
+                    "state and step results) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:
