@@ -162,7 +162,9 @@ int t2d_set_map_polygons(t2d_ctx* ctx, const float* segments, int n_seg, const i
 /* One tile = the static objects + boundary of one map (host arrays, copied).  tile_id: DEVICE uint16 [N], owned by the
  * caller and read by every tick: the tile of each scenario (may be rewritten between ticks, e.g. by a reset that draws a
  * new parking lot); NULL is allowed when n_tiles == 1.  Every scenario then collides with its own tile's objects, is
- * bounded by its own tile's box, and t2d_lidar_scan sees its own tile's segments. */
+ * bounded by its own tile's box, and t2d_lidar_scan sees its own tile's segments.
+ * A call that is rejected (any T2D_E_INVALID) changes nothing: the previous map stays in force, and with it the previous
+ * tile_id array, which the caller must keep alive until a later call succeeds. */
 #define T2D_MAX_TILES 4096
 typedef struct {
   const float* segments;     /* [n_seg][4] */

@@ -32,6 +32,7 @@
 
 #include "../../include/t2d_b200.h"
 #include "t2d_math.cuh"
+#include "t2d_tile.h"
 
 namespace t2d {
 
@@ -42,31 +43,6 @@ constexpr int MAX_WARPS_PER_CTA = T2D_K1_MAX_WARPS;
 constexpr int CTA_THREADS = MAX_WARPS_PER_CTA * 32;   // upper bound; the host picks the warps per CTA (pick_wpc)
 constexpr int POSE_PER_WARP = 128;      // 32 lanes x 4 participants per lane (PPL, template parameter of K1: 2 or 4)
 constexpr int MAP_SMEM_LIMIT = 120 * 1024;
-
-struct MapHeader {   // 128 bytes, start of a tile's blob
-  int32_t n_seg, gx, gy, n_items;
-  float x0, y0, inv_cell, cell;
-  uint32_t off_seg, off_cell, off_items, total_bytes;
-  uint32_t off_clear;   // float per cell: lower bound of the distance from any point of the cell to any segment
-  int32_t fine;         // the fine clearance field has (gx * fine) x (gy * fine) cells, one byte each (global memory)
-  // "dilated" lists: cell c lists (ascending) every segment that comes within `dil` metres of the cell's box, so that a
-  // participant whose bounding radius is <= dil finds all its candidates in the ONE cell under its centre (the grid
-  // covers the segments' bounding box grown by dil: a centre outside it cannot reach a segment)
-  uint32_t off_dcell, off_ditems;
-  float dil;
-  int32_t n_ditems;
-  uint32_t off_objfirst;   // uint16 per segment: first segment of the object (polygon / polyline piece) it belongs to
-  int32_t n_poly;          // closed rings among the segments (Area.geometry polygons)
-  uint32_t off_poly;       // int32 [n_poly + 1]: ring p = segments [start[p], start[p + 1])
-  uint32_t off_pbox;       // float4 per ring: xmin, xmax, ymin, ymax
-  uint32_t off_fine;       // the fine clearance field (bytes), last section of the blob
-  uint32_t smem_bytes;     // = off_fine: the part worth staging into shared memory
-  float bxmin, bxmax, bymin, bymax;   // Map.boundary of the tile (OutBound)
-  int32_t has_bounds;
-  uint32_t pad[3];
-};
-constexpr float CLEAR_QUANT = 0.125f;   // metres per unit of the byte-quantised fine clearance field
-static_assert(sizeof(MapHeader) == 128, "MapHeader must be 128 bytes");
 
 struct StepArgs {
   float *x, *y, *h, *v, *vx, *vy;
@@ -219,7 +195,7 @@ __device__ __noinline__ void other_model_step(OneIO& io, const Params& p, int n_
 
 // Static broadphase, level 1: the clearance field.  One shared-memory load tells whether the pose's
 // bounding circle can reach any segment at all (most participants are nowhere near a wall).
-// near_segments split in two so that the global byte load can be issued early and consumed late:
+// Split in two so that the global byte load can be issued early and consumed late:
 // near_fetch returns the quantised clearance under the participant (0 = treat as near: outside the grid but within
 // reach of it; 255 = far), near_decide compares it with the bounding radius.
 __device__ __forceinline__ unsigned near_fetch(const float ax, const float ay, const float rbound, const MapHeader& mh, const uint8_t* fine,
@@ -249,21 +225,6 @@ __device__ __forceinline__ unsigned near_fetch(const float ax, const float ay, c
 __device__ __forceinline__ bool near_decide(unsigned q, unsigned alt, const float rbound) {
   const unsigned v = alt == 0xffffffffu ? q : alt;
   return (float)v * CLEAR_QUANT <= rbound * 1.0001f + 1e-3f;
-}
-
-__device__ __forceinline__ bool near_segments(const float ax, const float ay, const float rbound, const MapHeader& mh,
-                                              const uint8_t* fine) {
-  const float r = rbound * 1.0001f + 1e-3f;
-  const float fx = (ax - mh.x0) * mh.inv_cell, fy = (ay - mh.y0) * mh.inv_cell;
-  const int gx = mh.gx, gy = mh.gy;
-  if (!(fx >= 0.0f && fy >= 0.0f && fx < (float)gx && fy < (float)gy)) {
-    // outside the grid: reachable only within r of its box
-    const float ox = fmaxf(fmaxf(-fx, fx - (float)gx), 0.0f), oy = fmaxf(fmaxf(-fy, fy - (float)gy), 0.0f);
-    return fmaxf(ox, oy) * mh.cell <= r;
-  }
-  const int k = mh.fine;
-  const int ix = min((int)(fx * (float)k), gx * k - 1), iy = min((int)(fy * (float)k), gy * k - 1);
-  return (float)__ldg(fine + (size_t)iy * (gx * k) + ix) * CLEAR_QUANT <= r;
 }
 
 // Own pose of participant `idx` back from the warp's shared-memory tile (the hot loops keep only x, y
@@ -400,24 +361,6 @@ __device__ __noinline__ void pair_exhaustive(int t0, int tb, int m0, int M, int 
 // of the warp's queue, counter qcount) and decided after the loop; if that queue is full the participant is
 // marked (returns -2) for the out-of-line exact walk.
 constexpr int QX0 = 128;   // first exact-queue entry (entries below hold the compacted participant list)
-
-// The sections of a map blob (in shared or in global memory: the accessors are inlined, the address space is known).
-struct MapView {
-  const float4* seg;
-  const uint32_t* cell_start;
-  const uint16_t* items;
-  const uint32_t* dcell_start;
-  const uint16_t* ditems;
-};
-__device__ __forceinline__ MapView map_view(const unsigned char* blob, const MapHeader& mh) {
-  MapView v;
-  v.seg = reinterpret_cast<const float4*>(blob + mh.off_seg);
-  v.cell_start = reinterpret_cast<const uint32_t*>(blob + mh.off_cell);
-  v.items = reinterpret_cast<const uint16_t*>(blob + mh.off_items);
-  v.dcell_start = reinterpret_cast<const uint32_t*>(blob + mh.off_dcell);
-  v.ditems = reinterpret_cast<const uint16_t*>(blob + mh.off_ditems);
-  return v;
-}
 
 // Static level 2 for ONE participant whose reach is <= the map's dilation: ONE cell look-up (the cell under the centre)
 // and one loop over its dilated list.  Returns the lowest hit, 0x7fffffff for none, -2 when the participant needs the
@@ -1950,221 +1893,28 @@ int t2d_set_type_table(t2d_ctx* c, const t2d_type_params* table, int n_types) {
   return T2D_OK;
 }
 
-// Host-side build of one static-geometry tile: the segments in list order (+ which of them close up to polygons), a
-// uniform grid over their bounding box grown by one cell, per cell the ascending list of the segments that touch it and
-// the "dilated" list of those within one cell of it, the clearance fields, the tile's boundary box.
-struct TileIn {
-  const float* segments; int n_seg;
-  const int32_t* poly_start; int n_poly;
-  const float* bounds;
-};
-
-static bool point_in_ring(const float* seg, int s0, int s1, double px, double py) {   // even-odd over the ring's edges
-  bool in = false;
-  for (int i = s0; i < s1; ++i) {
-    const double x1 = seg[4 * i], y1 = seg[4 * i + 1], x2 = seg[4 * i + 2], y2 = seg[4 * i + 3];
-    if ((y1 > py) != (y2 > py) && px < (x2 - x1) * (py - y1) / (y2 - y1) + x1) in = !in;
-  }
-  return in;
-}
-
-static int build_tile(const TileIn& t, float cell_size, float reach, std::vector<unsigned char>& blob) {
-  const float* segments = t.segments;
-  const int n_seg = t.n_seg;
-  if (n_seg < 0 || n_seg > T2D_MAX_SEGMENTS) return fail(T2D_E_INVALID, "n_seg must be in 0..32767");
-  if (n_seg > 0 && !segments) return fail(T2D_E_INVALID, "segments is NULL");
-  if (t.n_poly < 0 || (t.n_poly > 0 && !t.poly_start)) return fail(T2D_E_INVALID, "poly_start is NULL");
-  if (t.bounds && !(t.bounds[0] <= t.bounds[1] && t.bounds[2] <= t.bounds[3])) return fail(T2D_E_INVALID, "bounds must be (xmin<=xmax, ymin<=ymax)");
-  for (int p = 0; p < t.n_poly; ++p) {
-    const int s0 = t.poly_start[p], s1 = t.poly_start[p + 1];
-    if (s0 < 0 || s1 > n_seg || s1 - s0 < 3 || (p > 0 && s0 < t.poly_start[p])) return fail(T2D_E_INVALID, "poly_start: rings must be ascending, inside the segment list and have >= 3 edges");
-    for (int i = s0; i < s1; ++i) {   // a ring: every edge ends where the next one starts, the last one at the first one's start
-      const int j = i + 1 < s1 ? i + 1 : s0;
-      if (segments[4 * i + 2] != segments[4 * j] || segments[4 * i + 3] != segments[4 * j + 1]) return fail(T2D_E_INVALID, "poly_start: a ring's edges must chain and close");
-    }
-  }
-  MapHeader mh{};
-  mh.n_seg = n_seg; mh.n_poly = t.n_poly;
-  mh.has_bounds = t.bounds ? 1 : 0;
-  if (t.bounds) { mh.bxmin = t.bounds[0]; mh.bxmax = t.bounds[1]; mh.bymin = t.bounds[2]; mh.bymax = t.bounds[3]; }
-  if (n_seg == 0) {   // bounds only
-    mh.gx = mh.gy = 0; mh.total_bytes = mh.smem_bytes = mh.off_fine = sizeof(MapHeader);
-    blob.assign(sizeof(MapHeader), 0);
-    memcpy(blob.data(), &mh, sizeof(mh));
-    return T2D_OK;
-  }
-  float xmin = INFINITY, xmax = -INFINITY, ymin = INFINITY, ymax = -INFINITY;
-  for (int i = 0; i < n_seg * 4; ++i)
-    if (!std::isfinite(segments[i])) return fail(T2D_E_INVALID, "segments must be finite");
-  for (int i = 0; i < n_seg; ++i) {
-    const float* s = segments + 4 * i;
-    xmin = std::min(xmin, std::min(s[0], s[2])); xmax = std::max(xmax, std::max(s[0], s[2]));
-    ymin = std::min(ymin, std::min(s[1], s[3])); ymax = std::max(ymax, std::max(s[1], s[3]));
-  }
-  const float span = std::max(xmax - xmin, ymax - ymin);
-  float cell = cell_size > 0.0f ? cell_size : 8.0f;
-  // keep the grid small enough for shared memory: at most 64 x 64 cells over the box grown by one cell (the dilation)
-  while (span / cell > 62.0f) cell *= 2.0f;
-  // reach of the dilated lists: the largest bounding radius of the type table (as the kernel inflates it) when a table is
-  // set - shorter lists in dense maps - else one cell; a participant that reaches further takes the out-of-line walk
-  const float dil = reach > 0.0f ? std::min(cell, reach * 1.0002f + 2e-3f) : cell;
-  const float margin = 1e-3f * std::max(1.0f, std::max(std::fabs(xmin) + std::fabs(xmax), std::fabs(ymin) + std::fabs(ymax)) * 1e-3f);
-  const float x0 = xmin - dil - margin, y0 = ymin - dil - margin;
-  const int gx = std::max(1, (int)std::floor((xmax + dil + margin - x0) / cell) + 1);
-  const int gy = std::max(1, (int)std::floor((ymax + dil + margin - y0) / cell) + 1);
-  const float inv = 1.0f / cell;
-  // cells[c] lists (ascending) the segments that pass within `grow` of cell c's box (conservatively: the segment's line
-  // against the box grown by `grow` on every side)
-  auto bin_segments = [&](float grow) {
-    std::vector<std::vector<uint16_t>> cells((size_t)gx * gy);
-    for (int i = 0; i < n_seg; ++i) {
-      const float* s = segments + 4 * i;
-      const float g = grow + margin;
-      const float sx0 = std::min(s[0], s[2]) - g, sx1 = std::max(s[0], s[2]) + g;
-      const float sy0 = std::min(s[1], s[3]) - g, sy1 = std::max(s[1], s[3]) + g;
-      int cx0 = std::max(0, (int)std::floor((sx0 - x0) * inv)), cx1 = std::min(gx - 1, (int)std::floor((sx1 - x0) * inv));
-      int cy0 = std::max(0, (int)std::floor((sy0 - y0) * inv)), cy1 = std::min(gy - 1, (int)std::floor((sy1 - y0) * inv));
-      for (int cy = cy0; cy <= cy1; ++cy)
-        for (int cx = cx0; cx <= cx1; ++cx) {
-          // exact-enough cull: does the segment's line pass within the grown cell box?
-          const float bx0 = x0 + cx * cell - g, bx1 = x0 + (cx + 1) * cell + g;
-          const float by0 = y0 + cy * cell - g, by1 = y0 + (cy + 1) * cell + g;
-          const double dx = (double)s[2] - s[0], dy = (double)s[3] - s[1];
-          const double hx = 0.5 * ((double)bx1 - bx0), hy = 0.5 * ((double)by1 - by0);
-          const double mx = 0.5 * ((double)bx1 + bx0), my = 0.5 * ((double)by1 + by0);
-          const double cr = std::fabs(((double)s[0] - mx) * dy - ((double)s[1] - my) * dx);
-          if (cr > hx * std::fabs(dy) + hy * std::fabs(dx) + 1e-6 * (std::fabs(dx) + std::fabs(dy) + 1.0)) continue;
-          cells[(size_t)cy * gx + cx].push_back((uint16_t)i);
-        }
-    }
-    return cells;
-  };
-  const std::vector<std::vector<uint16_t>> cells = bin_segments(0.0f);
-  // the dilated lists serve participants with reach r <= dil from the cell under their centre: every segment within r
-  // of the centre is within dil of that cell's box (+ a 0.1 % + 1 mm guard for the fp32 cell index)
-  const std::vector<std::vector<uint16_t>> dcells = bin_segments(dil * 1.001f + 1e-3f);
-  size_t n_items = 0, n_ditems = 0;
-  for (auto& v : cells) n_items += v.size();
-  for (auto& v : dcells) n_ditems += v.size();
-  int fine = 4;   // bounded host work: cells x segments <= ~1e8 distance evaluations
-  while (fine > 1 && (double)gx * gy * fine * fine * n_seg > 1e8) fine >>= 1;
-  mh.gx = gx; mh.gy = gy; mh.n_items = (int)n_items; mh.n_ditems = (int)n_ditems; mh.fine = fine;
-  mh.x0 = x0; mh.y0 = y0; mh.inv_cell = inv; mh.cell = cell; mh.dil = dil;
-  auto up16 = [](size_t v) { return (v + 15) / 16 * 16; };
-  mh.off_seg = (uint32_t)up16(sizeof(MapHeader));
-  mh.off_cell = (uint32_t)up16(mh.off_seg + (size_t)n_seg * 16);
-  mh.off_items = (uint32_t)up16(mh.off_cell + ((size_t)gx * gy + 1) * 4);
-  mh.off_dcell = (uint32_t)up16(mh.off_items + n_items * 2);
-  mh.off_ditems = (uint32_t)up16(mh.off_dcell + ((size_t)gx * gy + 1) * 4);
-  mh.off_objfirst = (uint32_t)up16(mh.off_ditems + n_ditems * 2);
-  mh.off_poly = (uint32_t)up16(mh.off_objfirst + (size_t)n_seg * 2);
-  mh.off_pbox = (uint32_t)up16(mh.off_poly + ((size_t)t.n_poly + 1) * 4);
-  mh.off_clear = (uint32_t)up16(mh.off_pbox + (size_t)t.n_poly * 16);
-  mh.off_fine = (uint32_t)up16(mh.off_clear + (size_t)gx * gy * 4);
-  mh.smem_bytes = mh.off_fine;   // the fine field is read through L1 / L2, everything in front of it may be staged
-  mh.total_bytes = (uint32_t)up16(mh.off_fine + (size_t)gx * fine * gy * fine);
-  blob.assign(mh.total_bytes, 0);
-  memcpy(blob.data(), &mh, sizeof(mh));
-  memcpy(blob.data() + mh.off_seg, segments, (size_t)n_seg * 16);
-  auto write_lists = [&](const std::vector<std::vector<uint16_t>>& lists, uint32_t off_start, uint32_t off_items) {
-    uint32_t* cs = reinterpret_cast<uint32_t*>(blob.data() + off_start);
-    uint16_t* it = reinterpret_cast<uint16_t*>(blob.data() + off_items);
-    uint32_t acc = 0;
-    for (size_t ci = 0; ci < lists.size(); ++ci) {
-      cs[ci] = acc;
-      for (uint16_t sg : lists[ci]) it[acc++] = sg;
-    }
-    cs[lists.size()] = acc;
-  };
-  write_lists(cells, mh.off_cell, mh.off_items);
-  write_lists(dcells, mh.off_dcell, mh.off_ditems);
-  // the object a segment belongs to, named by the object's first segment: an open polyline piece is its own object, the
-  // edges of a polygon share the polygon's first edge (StaticCollision.update reports the first OBJECT hit, collision.py:37-43)
-  uint16_t* objfirst = reinterpret_cast<uint16_t*>(blob.data() + mh.off_objfirst);
-  for (int i = 0; i < n_seg; ++i) objfirst[i] = (uint16_t)i;
-  int32_t* pstart = reinterpret_cast<int32_t*>(blob.data() + mh.off_poly);
-  float* pbox = reinterpret_cast<float*>(blob.data() + mh.off_pbox);
-  for (int p = 0; p < t.n_poly; ++p) {
-    const int s0 = t.poly_start[p], s1 = t.poly_start[p + 1];
-    pstart[p] = s0;
-    float bx0 = INFINITY, bx1 = -INFINITY, by0 = INFINITY, by1 = -INFINITY;
-    for (int i = s0; i < s1; ++i) {
-      objfirst[i] = (uint16_t)s0;
-      bx0 = std::min(bx0, segments[4 * i]); bx1 = std::max(bx1, segments[4 * i]);
-      by0 = std::min(by0, segments[4 * i + 1]); by1 = std::max(by1, segments[4 * i + 1]);
-    }
-    pbox[4 * p] = bx0; pbox[4 * p + 1] = bx1; pbox[4 * p + 2] = by0; pbox[4 * p + 3] = by1;
-  }
-  pstart[t.n_poly] = t.n_poly > 0 ? t.poly_start[t.n_poly] : 0;
-  // clearance fields: lower bound of the distance from any point of a cell to the nearest segment
-  // (distance from the cell centre minus the half diagonal); ZERO inside a polygon - a pose deep inside an obstacle
-  // touches no edge but intersects the Area all the same.  Coarse (float per cell) and fine (bytes of CLEAR_QUANT metres,
-  // fine x fine per coarse cell, read through L1 / L2).
-  auto centre_dist = [&](double px, double py) {
-    for (int p = 0; p < t.n_poly; ++p)
-      if (px >= pbox[4 * p] && px <= pbox[4 * p + 1] && py >= pbox[4 * p + 2] && py <= pbox[4 * p + 3] &&
-          point_in_ring(segments, t.poly_start[p], t.poly_start[p + 1], px, py))
-        return 0.0;
-    double best = INFINITY;
-    for (int i = 0; i < n_seg; ++i) {
-      const float* sg = segments + 4 * i;
-      const double dx = (double)sg[2] - sg[0], dy = (double)sg[3] - sg[1], ux = px - sg[0], uy = py - sg[1];
-      const double dd = dx * dx + dy * dy;
-      double tt = dd > 0.0 ? (ux * dx + uy * dy) / dd : 0.0;
-      tt = std::min(1.0, std::max(0.0, tt));
-      const double ex = ux - tt * dx, ey = uy - tt * dy;
-      best = std::min(best, ex * ex + ey * ey);
-    }
-    return std::sqrt(best);
-  };
-  float* clr = reinterpret_cast<float*>(blob.data() + mh.off_clear);
-  {
-    const double half_diag = 0.5 * std::sqrt(2.0) * (double)cell * 1.0001 + 2.0 * margin;
-    for (int cy = 0; cy < gy; ++cy)
-      for (int cx = 0; cx < gx; ++cx) {
-        const double d = centre_dist((double)x0 + (cx + 0.5) * (double)cell, (double)y0 + (cy + 0.5) * (double)cell) - half_diag;
-        clr[(size_t)cy * gx + cx] = d > 0.0 ? (float)(d * 0.9999) : 0.0f;
-      }
-  }
-  uint8_t* fine_field = blob.data() + mh.off_fine;
-  {
-    const double fc = (double)cell / fine;
-    const double half_diag = 0.5 * std::sqrt(2.0) * fc * 1.001 + 2.0 * margin + 1e-3 * fc;
-    for (int iy = 0; iy < gy * fine; ++iy)
-      for (int ix = 0; ix < gx * fine; ++ix) {
-        const double d = centre_dist((double)x0 + (ix + 0.5) * fc, (double)y0 + (iy + 0.5) * fc) - half_diag;
-        const double q = std::floor(std::max(0.0, d) / CLEAR_QUANT);
-        fine_field[(size_t)iy * gx * fine + ix] = (uint8_t)std::min(255.0, q);
-      }
-  }
-  return T2D_OK;
-}
-
 int t2d_set_map_table(t2d_ctx* c, const t2d_map_tile* tiles, int n_tiles, const uint16_t* tile_id, float cell_size) {
   if (!c) return fail(T2D_E_INVALID, "ctx is NULL");
   if (n_tiles < 0 || n_tiles > T2D_MAX_TILES) return fail(T2D_E_INVALID, "n_tiles must be in 0..T2D_MAX_TILES");
   if (n_tiles > 0 && !tiles) return fail(T2D_E_INVALID, "tiles is NULL");
   if (n_tiles > 1 && !tile_id) return fail(T2D_E_INVALID, "tile_id is NULL (needed with more than one tile)");
+  // compiled before the current map is released: a rejected table leaves the current map in force
+  std::vector<unsigned char> all;
+  std::vector<uint32_t> offs;
+  std::string err;
+  if (int r = compile_map_table(tiles, n_tiles, cell_size, c->rb_max, all, offs, err)) return fail(r, err);
   CUDA_TRY(cudaSetDevice(c->device));
   if (c->d_map) { cudaFree(c->d_map); c->d_map = nullptr; }
   if (c->d_tile_off) { cudaFree(c->d_tile_off); c->d_tile_off = nullptr; }
   c->map_bytes = 0; c->n_tiles = 0; c->tile_id = nullptr; c->has_bounds = false; c->has_segments = false;
   c->mh = MapHeader{};
   if (n_tiles == 0) return T2D_OK;
-  std::vector<unsigned char> all;
-  std::vector<uint32_t> offs((size_t)n_tiles);
   bool any_bounds = false, any_seg = false;
   for (int i = 0; i < n_tiles; ++i) {
-    TileIn t{tiles[i].segments, tiles[i].n_seg, tiles[i].poly_start, tiles[i].n_poly, tiles[i].bounds};
-    std::vector<unsigned char> blob;
-    if (int r = build_tile(t, cell_size, c->rb_max, blob)) return r;
-    offs[i] = (uint32_t)all.size();
-    all.insert(all.end(), blob.begin(), blob.end());
-    all.resize((all.size() + 127) / 128 * 128, 0);   // every tile starts 128-byte aligned
     any_bounds = any_bounds || tiles[i].bounds != nullptr;
     any_seg = any_seg || tiles[i].n_seg > 0;
-    if (i == 0) memcpy(&c->mh, blob.data(), sizeof(MapHeader));
   }
+  memcpy(&c->mh, all.data(), sizeof(MapHeader));   // tile 0 starts at offset 0
   CUDA_TRY(cudaMalloc(&c->d_map, all.size()));
   CUDA_TRY(cudaMemcpy(c->d_map, all.data(), all.size(), cudaMemcpyHostToDevice));
   CUDA_TRY(cudaMalloc(&c->d_tile_off, sizeof(uint32_t) * (size_t)n_tiles));

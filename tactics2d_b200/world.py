@@ -183,8 +183,10 @@ class BatchedWorld:
         tid = torch.as_tensor(np.asarray(tile_id) if not torch.is_tensor(tile_id) else tile_id).to(torch.int64)
         if tid.numel() != self.N or int(tid.min()) < 0 or int(tid.max()) >= len(tiles):
             raise ValueError(f"tile_id must hold {self.N} indices into the {len(tiles)} tiles")
-        self.tile_id = tid.to(torch.int16).to(self.device).contiguous()   # (bit pattern of uint16 for ids < 32768)
-        _lib.check(self.lib.t2d_set_map_table(self._ctx, rows, len(tiles), _ptr(self.tile_id), float(cell_size)))
+        tid = tid.to(torch.int16).to(self.device).contiguous()   # (bit pattern of uint16 for ids < 32768)
+        # a rejected table leaves the previous map, and the ids it reads, in force: replace self.tile_id only on success
+        _lib.check(self.lib.t2d_set_map_table(self._ctx, rows, len(tiles), _ptr(tid), float(cell_size)))
+        self.tile_id = tid
         self.tiles = [dict(segments=k[0], bounds=None if k[1] is None else tuple(float(v) for v in k[1]), poly_start=k[2]) for k in keep]
         self.segments, self.poly_start, self.bounds = None, None, None
 

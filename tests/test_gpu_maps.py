@@ -5,24 +5,9 @@ import numpy as np
 import pytest
 
 from oracle import scenario as O
+from tests.util import parking_like_objects
 
 pytestmark = pytest.mark.gpu
-
-
-def _parking_like_objects():
-    """Walls and obstacles the way ParkingLotGenerator builds them (map/generator/generate_parking_lot.py:122-205,354-385):
-    Area polygons - a long wall, a block big enough to swallow a car, an L-shaped (concave) obstacle, a kerb stone smaller
-    than a car - plus an open kerb line."""
-    from tactics2d_b200.map import polygons_to_segments
-
-    polys = [
-        [(-30, 18), (30, 18), (30, 19), (-30, 19)],                          # wall
-        [(-25, -20), (-5, -20), (-5, -4), (-25, -4)],                        # block: a car fits inside
-        [(4, -18), (16, -18), (16, -6), (12, -6), (12, -14), (4, -14)],      # L shape: its notch is outside the polygon
-        [(20.0, 5.0), (20.8, 5.0), (20.8, 5.4), (20.0, 5.4)],                # smaller than a car
-    ]
-    lines = [[(-30, -26), (0, -27), (30, -26)]]
-    return polygons_to_segments(polys, lines)
 
 
 def test_polygon_obstacles_containment_and_first_object(cuda_device):
@@ -30,7 +15,7 @@ def test_polygon_obstacles_containment_and_first_object(cuda_device):
 
     from tactics2d_b200 import BatchedWorld, synthetic
 
-    seg, ps = _parking_like_objects()
+    seg, ps = parking_like_objects()
     bounds = (-40.0, 40.0, -40.0, 40.0)
     n, m = 96, 16
     scene = synthetic.config2(n, m, seed=41, size=70.0)
@@ -73,6 +58,59 @@ def test_polygon_obstacles_containment_and_first_object(cuda_device):
     w.close()
 
 
+def test_rejected_map_leaves_the_previous_map_in_force(cuda_device):
+    """A set_map or set_map_table whose tile the compiler rejects changes nothing: the world keeps colliding with the map,
+    and reading the tile ids, it had."""
+    import torch
+
+    from tactics2d_b200 import BatchedWorld, synthetic
+    from tactics2d_b200._lib import T2DError
+
+    seg, ps = parking_like_objects()
+    bounds = (-40.0, 40.0, -40.0, 40.0)
+    n, m = 32, 16
+    scene = synthetic.config2(n, m, seed=47, size=70.0)
+    x, y = scene.x - 35.0, scene.y - 35.0
+    table = scene.table.as_oracle_table()
+    w = BatchedWorld(n, m, scene.table, device=cuda_device, any_participant=True)
+    w.set_map(seg, bounds, poly_start=ps)
+    w.set_state(x, y, scene.heading, scene.speed, type_id=scene.type_id)
+    fl, hi, hs = O.events(x, y, scene.heading, scene.type_id, table, seg, bounds, poly_start=ps)
+    assert ((fl & 2) != 0).sum() > 0
+
+    def check():
+        r = w.check_events()
+        torch.cuda.synchronize()
+        assert np.array_equal(r.flags.cpu().numpy(), fl)
+        assert np.array_equal(r.hit_segment.cpu().numpy(), hs) and np.array_equal(r.hit_index.cpu().numpy(), hi)
+
+    check()
+    open_ring = np.array([[0, 0, 4, 0], [4, 0, 4, 4], [4, 4, 0, 4], [0, 4, 0, 1]], np.float32)   # does not close
+    with pytest.raises(T2DError, match="chain and close"):
+        w.set_map(open_ring, (-10.0, 10.0, -10.0, 10.0), poly_start=[0, 4])
+    check()
+    # the same for a table: a rejected set_map_table keeps the previous tiles and the tile ids they are read with
+    tiles = [dict(segments=seg, bounds=bounds, poly_start=ps), dict(segments=seg, bounds=(-30.0, 30.0, -30.0, 30.0), poly_start=None)]
+    per_tile = [O.events(x, y, scene.heading, scene.type_id, table, t["segments"], t["bounds"], poly_start=t["poly_start"]) for t in tiles]
+    ids = np.arange(n) % 2
+
+    def expected(ids):
+        return [np.where(ids[:, None] == 1, a1, a0) for a0, a1 in zip(*per_tile)]
+
+    w.set_map_table(tiles, ids)
+    fl, hi, hs = expected(ids)
+    assert not np.array_equal(fl, expected(1 - ids)[0])
+    check()
+    with pytest.raises(T2DError, match="chain and close"):
+        w.set_map_table([tiles[0], dict(segments=open_ring, bounds=None, poly_start=[0, 4])], 1 - ids)
+    assert np.array_equal(w.tile_id.cpu().numpy(), ids)
+    # id arrays of the same size allocated now would reuse the memory of a dropped one: they hold valid ids, the wrong ones
+    filler = [torch.from_numpy((1 - ids).astype(np.int16)).to(cuda_device) for _ in range(4)]
+    check()
+    del filler
+    w.close()
+
+
 def test_map_table_one_tile_per_scenario(cuda_device):
     """configs[2] says "highD_map tiles": highD_1 .. highD_6 in ONE batch, every scenario on its own tile (segments and
     boundary box), plus a tile of polygons and an empty tile; tile ids rewritten between ticks."""
@@ -85,7 +123,7 @@ def test_map_table_one_tile_per_scenario(cuda_device):
     for k in range(1, 7):
         seg, bounds = load_collidable_segments(f"highD_{k}")
         tiles.append(dict(segments=seg, bounds=bounds, poly_start=None))
-    pseg, ps = _parking_like_objects()
+    pseg, ps = parking_like_objects()
     tiles.append(dict(segments=pseg, bounds=(-40.0, 40.0, -40.0, 40.0), poly_start=ps))
     tiles.append(dict(segments=None, bounds=(0.0, 100.0, -50.0, 50.0), poly_start=None))       # bounds only
     n, m = 64, 32

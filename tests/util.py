@@ -34,3 +34,19 @@ def assert_state_close(got: dict, ref: dict, mask=None, rtol=RTOL, what=""):
     bad = {k: v for k, v in worst.items() if not v <= rtol}
     assert not bad, f"{what} state mismatch beyond {rtol}: {bad} (all: {worst})"
     return worst
+
+
+def parking_like_objects():
+    """Walls and obstacles the way ParkingLotGenerator builds them (map/generator/generate_parking_lot.py:122-205,354-385):
+    Area polygons - a long wall, a block big enough to swallow a car, an L-shaped (concave) obstacle, a kerb stone smaller
+    than a car - plus an open kerb line."""
+    from tactics2d_b200.map import polygons_to_segments
+
+    polys = [
+        [(-30, 18), (30, 18), (30, 19), (-30, 19)],                          # wall
+        [(-25, -20), (-5, -20), (-5, -4), (-25, -4)],                        # block: a car fits inside
+        [(4, -18), (16, -18), (16, -6), (12, -6), (12, -14), (4, -14)],      # L shape: its notch is outside the polygon
+        [(20.0, 5.0), (20.8, 5.0), (20.8, 5.4), (20.0, 5.4)],                # smaller than a car
+    ]
+    lines = [[(-30, -26), (0, -27), (30, -26)]]
+    return polygons_to_segments(polys, lines)
